@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — decode tok/s of the quantized-MoE hot path at DeepSeek-V3 shapes.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config.workload): DeepSeek-V3 671B Q4_K_M single-stream decode, the MoE-block hot path of every
@@ -394,9 +394,8 @@ def full_decode_leg(args, lib, native, dev, local_rank, layers, L, moe_layer_cal
         e1.record(); torch.cuda.synchronize()
         return e0.elapsed_time(e1) / steps, launches
 
-    steps = max(5, min(args.steps, 20))
-    ms_full, launches = timed(lambda: step(True, True), steps)
-    ms_noattn, _ = timed(lambda: step(True, False), steps)
+    ms_full, launches = timed(lambda: step(True, True), args.steps)
+    ms_noattn, _ = timed(lambda: step(True, False), args.steps)
     attn_bytes = NL * ((H * QL + H * (KVL + ROPE) + QL * NH * (NOPE + ROPE) + NH * VD * H) * 144 // 256 + 2 * NH * NOPE * KVL * 2 + (ctx + 1) * (KVL + ROPE) * 2)
     moe_bytes = N_MOE_LAYERS * ((K + 1) * BYTES_PER_EXPERT + E * H * 4) // (1 if world == 1 else 1)
     other_bytes = 3 * (2 * DI * H * 144 // 256 + H * DI * 210 // 256) + VOCAB * H * 210 // 256
@@ -423,7 +422,14 @@ def main():
     ap.add_argument("--ctx", type=int, default=4096, help="cached tokens per sequence in the whole-step leg")
     ap.add_argument("--no-full-step", action="store_true")
     ap.add_argument("--no-prefill", action="store_true", help="skip the 1024-token grouped-GEMM leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy: the MoE block output, routed ids "
+                         "and weights of its last layer (every layer of a step writes the same buffers)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the b200 arm")
     # This process owns the GPU and decodes on ONE stream: the persistent MoE-block kernel is launched as a plain grid
     # with programmatic dependent launch (its 148 CTAs become co-resident as the previous layer's CTAs exit) instead of
     # cooperatively — the cooperative attribute (library default: safe when several streams share the GPU) makes every
@@ -574,8 +580,8 @@ def main():
 
     rng = np.random.default_rng(1234 + rank)
 
-    def fresh_input():
-        x_host.copy_(torch.from_numpy((rng.standard_normal((1, H)) / 100).astype(np.float32)).to(torch.bfloat16))
+    def fresh_input(gen=rng):
+        x_host.copy_(torch.from_numpy((gen.standard_normal((1, H)) / 100).astype(np.float32)).to(torch.bfloat16))
 
     # ---- parity check (outside every timed region): layer 0's output for this step's token against the CPU oracle ------
     parity = None
@@ -690,7 +696,8 @@ def main():
         run_step(); torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
-    fresh_input(); x_own.copy_(x_host); barrier()
+    # the timed token has a generator of its own: it does not depend on how many draws the parity check and warm-up took
+    fresh_input(np.random.default_rng(4321 + rank)); x_own.copy_(x_host); barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
@@ -704,6 +711,14 @@ def main():
         dist.all_reduce(t_ms, op=dist.ReduceOp.MAX)
     ms_per_step = float(t_ms.item()) / args.steps
     value = world * 1000.0 / ms_per_step
+
+    # ---- the last timed step's outputs, for comparing two builds on the same seeded inputs --------------------------------
+    # Every layer of a step reads the same token and writes these buffers, so they hold what the step's last layer returned.
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in (("moe_out", y.float().cpu().numpy()), ("topk_ids", ids.cpu().numpy().astype(np.float64)),
+                          ("topk_weights", wts.cpu().numpy())):
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
 
     # ---- e2e: host buffers, copies inside the timed region ----------------------------------------------------
     if world == 1:

@@ -33,6 +33,17 @@ def golden_dir():
 
 
 @pytest.fixture(scope="session")
+def moe_small(golden_dir):
+    """The reference's MOE::forward fixture (tests/golden/make_golden.py), stored in parts of under 1 MB each."""
+    import numpy as np
+    out = {}
+    for part in ("gate", "up", "down", "io"):
+        with np.load(os.path.join(golden_dir, f"moe_small_{part}.npz")) as g:
+            out.update({k: g[k] for k in g.files})
+    return out
+
+
+@pytest.fixture(scope="session")
 def oracle():
     from oracle.bindings import Oracle
     return Oracle()

@@ -5,7 +5,7 @@ reference's Python.  Run in the build container only:
     make -C oracle ref && python tests/golden/make_golden.py
 
 Outputs (small, committed):
-    moe_small.npz        E=4 k=2 H=512 I=256, Q4_K/Q4_K/Q6_K + a Q5_K/Q5_K/Q4_K variant: quantised weights
+    moe_small_*.npz      E=4 k=2 H=512 I=256, Q4_K/Q4_K/Q6_K + a Q5_K/Q5_K/Q4_K variant: quantised weights
                          (reference from_float), inputs, MOE::forward outputs for qlen 1,3,12 (fp32 and bf16)
     act_quant.npz        Q8_K / Q8_0 activation blocks for fp32 and bf16-valued rows (tie-heavy)
     dequant.npz          16 blocks per weight type: raw bytes + to_float values
@@ -51,7 +51,12 @@ def moe_case(rng, E, k, H, I, gt, ut, dt, qlens):
 rng = np.random.default_rng(20260922)
 a = moe_case(rng, 4, 2, 512, 256, Q4_K, Q4_K, Q6_K, (1, 3, 12))
 b = moe_case(rng, 4, 2, 512, 256, Q5_K, Q5_K, Q4_K, (1, 12))
-np.savez_compressed(os.path.join(OUT, "moe_small.npz"), **{f"a_{k}": v for k, v in a.items()}, **{f"b_{k}": v for k, v in b.items()})
+moe = {**{f"a_{k}": v for k, v in a.items()}, **{f"b_{k}": v for k, v in b.items()}}
+# one file per weight tensor plus one for the rest, so that no file exceeds 1 MB; tests/conftest.py joins them again
+for part in ("gate", "up", "down"):
+    np.savez_compressed(os.path.join(OUT, f"moe_small_{part}.npz"), **{n: v for n, v in moe.items() if n.endswith("_" + part)})
+np.savez_compressed(os.path.join(OUT, "moe_small_io.npz"),
+                    **{n: v for n, v in moe.items() if not n.endswith(("_gate", "_up", "_down"))})
 
 # activation quantisation
 rows = []

@@ -85,8 +85,8 @@ def test_dequantise_vs_golden(golden_dir, name):
 
 # ------------------------------------------------------------------------------------------ MoE vs golden
 @pytest.mark.parametrize("case", ["a", "b"])
-def test_moe_forward_vs_golden(golden_dir, case):
-    g = np.load(os.path.join(golden_dir, "moe_small.npz"))
+def test_moe_forward_vs_golden(moe_small, case):
+    g = moe_small
     E, k, H, I = (int(g[f"{case}_{n}"]) for n in ("E", "k", "H", "I"))
     gt, ut, dt = (int(g[f"{case}_{n}"]) for n in ("gate_type", "up_type", "down_type"))
     for hid in (F32, BF16):
